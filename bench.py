@@ -11,9 +11,10 @@ A STEP = one pass of the hot path over one scheduler batch of 64 single-row requ
   e2e     the same batch through the C ABI with HOST buffers: b2s_infer_batch (collate into the pinned
           slot, H2D, kernel, result written back to the host) + b2s_event_wait (scatter to the 64
           per-request buffers), wall clock, up to 4 batches in flight
-  Every timed leg REPEATS its K-step region until it has accumulated >= MIN_TIMED_S of timed work and at least
-  MIN_REPEATS repeats, and reports the MEDIAN region (a 20-step region of this workload is 0.3 ms: one scheduler
-  hiccup on one rank used to decide the whole-job number).
+  Every forest leg times exactly K steps, once, after an untimed warm-up in its own step form (>= W steps and
+  >= WARMUP_MIN_S); step k reads input set k % 64, so the inputs of the last timed step depend on K alone, and
+  --dump-outputs DIR writes what that step of `value` returned.  A small K is a noisy figure (a 20-step region of this
+  workload is 0.3 ms).
   plugin  the metric BASELINE.json names, through the reference-facing plugin API
           (B200PreprocessRequest.process under asyncio): closed-loop req/s and open-loop Poisson
           (lambda = 2000 req/s) p50/p99 latency
@@ -43,14 +44,16 @@ WORKLOAD_MIN_STEPS = 200     # BERT / ResNet sections: timed steps whatever --st
 # the ResNet loop ran at 3.38 ms per batch against 2.93 ms on the device (collate + H2D of batch k+2 not hidden); 3: 2.96; 4: 2.74
 WORKLOAD_E2E_DEPTH = int(os.environ.get("B2S_BENCH_E2E_DEPTH", "4"))
 MIN_TIMED_S, MIN_REPEATS, MAX_LEG_WALL_S = 0.5, 5, 25.0
+# a single K-step region timed right after a 50-step warm-up ran the e2e leg 25 % slower than the steady state
+# (B200, 1000 W power limit, K = 500)
+WARMUP_MIN_S = 0.5
 
 
 def _config():
     """the `config` object: identical in both arms (the driver compares them)"""
     return dict(workload=WORKLOAD, step="one scheduler batch of 64 single-row requests", max_batch=MAX_BATCH,
                 n_trees=N_TREES, depth=DEPTH, n_features=N_FEATURES,
-                timing="K-step region repeated until >= {} s of timed work and >= {} repeats; median region".format(
-                    MIN_TIMED_S, MIN_REPEATS),
+                timing="exactly K timed steps (--steps), one region, after an untimed warm-up",
                 l2="GPU arm: flushed (256 MiB memset on the launching stream) before every timed step of `value`")
 
 
@@ -64,6 +67,15 @@ def _repeat_region(region, min_timed_s=MIN_TIMED_S, min_repeats=MIN_REPEATS, max
         if time.perf_counter() - t0 > max_wall_s and len(samples) >= min_repeats:
             break
     return float(np.median(samples)), samples
+
+
+def _warm_up(run, n):
+    """Untimed warm-up of a leg in its own step form: run(n) runs n steps; repeated until WARMUP_MIN_S have passed, so
+    that clocks and host caches have settled before the leg's K timed steps, whatever W is."""
+    t0 = time.perf_counter()
+    run(n)
+    while time.perf_counter() - t0 < WARMUP_MIN_S:
+        run(n)
 
 
 def _peaks():
@@ -189,6 +201,18 @@ def _sum_over_ranks(dist, local, x):
     return float(t.item())
 
 
+def _dump_outputs(out_dir, **arrays):
+    """--dump-outputs: each array as <out_dir>/<name>.npy (float32 / float64), for output-for-output comparison of
+    two builds run with the same arguments"""
+    if not out_dir:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def whole_job_value(world, units_per_rank_per_step, steps, max_seconds):
     """`value` of the contract: units all ranks processed / the slowest rank's time (weak scaling)."""
     return world * units_per_rank_per_step * steps / max_seconds
@@ -226,8 +250,9 @@ def _cpu_pick_threads(h, X, out, n_procs):
 
 def _cpu_loop(forest, steps, warmup=3):
     """The oracle port (no compiled reference exists: clearml-serving is pure Python and xgboost is not installable) on
-    the host cores: one step = one batch of 64 rows, OpenMP over rows with the fastest team size the box offers.  The
-    K-step region is repeated like the GPU legs.  Returns (median seconds per region, repeats, threads, n_procs, sweep)."""
+    the host cores: one step = one batch of 64 rows, OpenMP over rows with the fastest team size the box offers.
+    Returns (region, out, threads, n_procs, sweep): region() times `steps` steps, step k on input set k % 256, and
+    leaves the last step's predictions in `out`."""
     from oracle import oracle as orc
     h = orc.ForestHandle(forest)
     n_procs = orc.max_threads()
@@ -237,21 +262,21 @@ def _cpu_loop(forest, steps, warmup=3):
     threads, sweep = _cpu_pick_threads(h, X, out, n_procs)
     for w in range(warmup):
         h.predict_xgb_into(X[w % 256], 0.5, out, threads)
-    k = [0]
 
     def region():
         t0 = time.perf_counter()
-        for _ in range(steps):
-            h.predict_xgb_into(X[k[0] % 256], 0.5, out, threads)
-            k[0] += 1
+        for k in range(steps):
+            h.predict_xgb_into(X[k % 256], 0.5, out, threads)
         return time.perf_counter() - t0
-    med, samples = _repeat_region(region)
-    return med, len(samples), threads, n_procs, sweep
+    return region, out, threads, n_procs, sweep
 
 
 def _cpu_baseline(forest, seconds):
+    """comparison leg, independent of --steps: its 200-step region is repeated (_repeat_region), median region"""
     steps = 200
-    med, reps, threads, n_procs, sweep = _cpu_loop(forest, steps)
+    region, _out, threads, n_procs, sweep = _cpu_loop(forest, steps)
+    med, samples = _repeat_region(region)
+    reps = len(samples)
     return dict(value=steps * MAX_BATCH / med, unit="requests/s", cores=int(threads), kind="port",
                 sample="median of {} regions of {} batches x {} rows; oracle/forest_oracle.c (restatement of the xgboost "
                        "CPU predictor), OpenMP over rows, team size {} of {} host threads (fixed sweep, finalists re-timed "
@@ -355,16 +380,18 @@ def run_reference(args):
         return
     forest = _make_model()
     W = max(args.warmup, 3)
-    med, reps, threads, n_procs, sweep = _cpu_loop(forest, args.steps, warmup=W)
-    value = args.steps * MAX_BATCH / med
+    region, out, threads, n_procs, sweep = _cpu_loop(forest, args.steps, warmup=W)
+    secs = region()
+    _dump_outputs(args.dump_outputs, forest_predictions=out)
+    value = args.steps * MAX_BATCH / secs
     line = dict(metric="requests/sec", value=value, unit="requests/s", n_gpus=args.gpus, steps=args.steps,
-                warmup=W, ms_per_step=med / args.steps * 1e3, higher_is_better=True, scaling="weak",
-                vs_baseline=None, dtype="f32", data="synthetic", impl="reference", repeats=reps,
+                warmup=W, ms_per_step=secs / args.steps * 1e3, higher_is_better=True, scaling="weak",
+                vs_baseline=None, dtype="f32", data="synthetic", impl="reference",
                 config=_config(),
                 cpu_baseline=dict(value=value, unit="requests/s", cores=int(threads), kind="port",
-                                  sample="median of {} regions of {} steps x {} rows; oracle port of the xgboost CPU predictor, "
+                                  sample="one region of {} steps x {} rows; oracle port of the xgboost CPU predictor, "
                                          "OpenMP over rows, team size {} of {} host threads (fixed sweep, finalists re-timed "
-                                         "for 1 s)".format(reps, args.steps, MAX_BATCH, threads, n_procs),
+                                         "for 1 s)".format(args.steps, MAX_BATCH, threads, n_procs),
                                   team_sweep_req_s={str(k): round(v) for k, v in sorted(sweep.items())}),
                 e2e=dict(value=value, unit="requests/s", h2d_bytes_per_step=0, d2h_bytes_per_step=0))
     print(json.dumps(line))
@@ -1088,39 +1115,35 @@ def run_b200(args):
     for b, x in zip(d_in, Xs):
         b.upload(x)
     d_out = native.DeviceBuffer(MAX_BATCH * 4, device)
-    for w in range(W):
-        stream.infer_device(MAX_BATCH, [d_in[w % n_sets].ptr], [d_out.ptr])
-    stream.synchronize()
 
-    clocks = ClockSampler(device)
-    launches0 = native.launch_count()
-    step_no = [0]
-
-    def cold_region():
+    # step k of every region reads input set k % n_sets: the last timed step's inputs depend on K alone
+    def cold_region(n):
         ms = 0.0
-        for _ in range(K):
+        for k in range(n):
             stream.flush_l2()                      # untimed, same stream: evict model + inputs from the 126 MB L2
             timer.start()
-            stream.infer_device(MAX_BATCH, [d_in[step_no[0] % n_sets].ptr], [d_out.ptr])
+            stream.infer_device(MAX_BATCH, [d_in[k % n_sets].ptr], [d_out.ptr])
             timer.stop()
             ms += timer.elapsed_ms()
-            step_no[0] += 1
         return ms * 1e-3
 
     def warm_region():   # same launches back to back, model resident in L2 (steady-state serving)
         timer.start()
-        for _ in range(K):
-            stream.infer_device(MAX_BATCH, [d_in[step_no[0] % n_sets].ptr], [d_out.ptr])
-            step_no[0] += 1
+        for k in range(K):
+            stream.infer_device(MAX_BATCH, [d_in[k % n_sets].ptr], [d_out.ptr])
         timer.stop()
         return timer.elapsed_ms() * 1e-3
+    _warm_up(cold_region, W)
+
+    clocks = ClockSampler(device)
+    launches0 = native.launch_count()
     _barrier_sync(dist, local)
-    cold_s, cold_samples = _repeat_region(cold_region)
+    cold_s = cold_region(K)
     stream.synchronize()
+    last_out = d_out.download(np.float32, MAX_BATCH)   # what the last timed step returned
     _barrier_sync(dist, local)
     cold_s = _max_over_ranks(dist, local, cold_s)
-    warm_s, _ws = _repeat_region(warm_region)
-    warm_s = _max_over_ranks(dist, local, warm_s)
+    warm_s = _max_over_ranks(dist, local, warm_region())
     kernel_launches = native.launch_count() - launches0
 
     # ---------------------------------------------------------------- e2e: C ABI with host buffers
@@ -1155,12 +1178,12 @@ def run_b200(args):
             native.check(lib.b2s_event_wait(ev))
         return time.perf_counter() - t0
 
-    e2e_run(max(W, 50), 4)
+    _warm_up(lambda n: e2e_run(n, 4), max(W, 50))
     _barrier_sync(dist, local)
-    e2e_s, e2e_samples = _repeat_region(lambda: e2e_run(K, 4))
-    e2e_s = _max_over_ranks(dist, local, e2e_s)
-    e2e_lat_s, _ls = _repeat_region(lambda: e2e_run(K, 1))
-    e2e_lat_s = _max_over_ranks(dist, local, e2e_lat_s)
+    e2e_s = _max_over_ranks(dist, local, e2e_run(K, 4))
+    _warm_up(lambda n: e2e_run(n, 1), max(W, 50))
+    _barrier_sync(dist, local)
+    e2e_lat_s = _max_over_ranks(dist, local, e2e_run(K, 1))
     _barrier_sync(dist, local)
     launches = native.launch_count() - launches0
 
@@ -1230,6 +1253,7 @@ def run_b200(args):
                 raise
 
     if rank == 0:
+        _dump_outputs(args.dump_outputs, forest_predictions=last_out)
         peak, peak_src = _peaks()
         algo = model.algo_bytes(MAX_BATCH)
         kernel_s = cold_s / K
@@ -1251,13 +1275,13 @@ def run_b200(args):
         line = dict(
             metric="requests/sec", value=value, unit="requests/s", n_gpus=world, steps=K, warmup=W,
             ms_per_step=cold_s / K * 1e3, higher_is_better=True, scaling="weak", vs_baseline=None,
-            dtype="f32", data="synthetic", config=cfg, repeats=len(cold_samples),
-            timed_region_s=dict(value=float(np.sum(cold_samples)), e2e=float(np.sum(e2e_samples))),
+            dtype="f32", data="synthetic", config=cfg,
+            timed_region_s=dict(value=cold_s, e2e=e2e_s),
             notes=dict(l2="flushed (256 MiB memset on the launching stream) before every timed step; value_l2_warm is the "
                           "back-to-back figure", parallelism="replicas x{} (independent requests, no collective)".format(world)),
             value_l2_warm=world * MAX_BATCH * K / warm_s, ms_per_step_l2_warm=warm_s / K * 1e3,
             e2e=dict(value=world * MAX_BATCH * K / e2e_s, unit="requests/s", h2d_bytes_per_step=MAX_BATCH * N_FEATURES * 4,
-                     d2h_bytes_per_step=MAX_BATCH * 4, ms_per_step=e2e_s / K * 1e3, in_flight=4, repeats=len(e2e_samples),
+                     d2h_bytes_per_step=MAX_BATCH * 4, ms_per_step=e2e_s / K * 1e3, in_flight=4,
                      ms_per_step_serial=e2e_lat_s / K * 1e3,
                      path="b2s_infer_batch(64 host tensors) + b2s_event_wait, wall clock"),
             gpu_launches=int(launches), gpu_launches_value_leg=int(kernel_launches),
@@ -1290,6 +1314,9 @@ def main():
     ap.add_argument("--no-bert", dest="bert", action="store_false", help="skip the BERT-base (configs[3]) section")
     ap.add_argument("--no-resnet", dest="resnet", action="store_false", help="skip the ResNet-50 (configs[2]) section")
     ap.add_argument("--no-llama", dest="llama", action="store_false", help="skip the Llama-3-8B (configs[4]) section")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the predictions of the last timed step of `value` (64 rows, float32) to "
+                         "DIR/forest_predictions.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

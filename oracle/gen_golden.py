@@ -17,6 +17,8 @@ Fixtures
                        shapes and decoded outputs for the marshalling edge cases
   rest_contract.json   the reference FastAPI app (main.py) under starlette TestClient:
                        request -> (status, body) pairs incl. 404/422 detail strings
+  reference_dropin.json the b200 engine registered into the reference's registry by integration.register_with_reference
+                       and served by the reference's ModelRequestProcessor.process_request: the replies, per engine name
 """
 import asyncio
 import gzip
@@ -164,6 +166,8 @@ def gen_trees_cfg2(ref):
     init = float(gbr.init_.constant_.ravel()[0])
     compact = dict(forest)
     compact["feat"] = forest["feat"].astype(np.int16)
+    # internal-node values are never read (only leaves carry an output): stored as 0, which keeps the file under 1 MB
+    compact["value"] = np.where(forest["left"] < 0, forest["value"], 0.0)
     np.savez_compressed(os.path.join(GOLD, "sk_gbr_cfg2.npz"), X=X, y=y, init=init, scale=float(gbr.learning_rate),
                         divisor=1.0, **compact)
     chk = orc.forest_predict_f64(forest, X, init, float(gbr.learning_rate), 1.0)
@@ -281,6 +285,21 @@ def gen_rest(ref, lr_model):
         json.dump(out, f, indent=1)
 
 
+def gen_dropin(ref):
+    """tests/test_reference_dropin.py's scenario through the reference's own dispatcher, per engine name"""
+    import tempfile
+    import pytest
+    from tests import test_reference_dropin as t
+    out = {}
+    for name in t.ENGINE_NAMES:
+        with pytest.MonkeyPatch.context() as mp, tempfile.TemporaryDirectory() as tmp:
+            made = t.install_fake_native(mp)
+            out[name] = t.serve(t.reference_dispatcher(ref), name, tmp, made)
+    with open(os.path.join(GOLD, "reference_dropin.json"), "w") as f:
+        json.dump(out, f, indent=1)
+    print("reference_dropin:", {k: len(v["replies"]) for k, v in out.items()})
+
+
 def main():
     os.makedirs(GOLD, exist_ok=True)
     ref = rh.load_reference()
@@ -289,6 +308,7 @@ def main():
     gen_trees_cfg2(ref)
     gen_triton_marshal(ref)
     gen_rest(ref, lr)
+    gen_dropin(ref)
 
 
 if __name__ == "__main__":
