@@ -1635,7 +1635,7 @@ extern "C" B2S_API int b2s_op_gemm(int device, void *cuda_stream, const void *A,
     ep.bias = bias;
     ep.residual = residual;
     ep.C = C;
-    ep.ldc = N;
+    ep.ldc = act == 4 ? N / 2 : N;   // ACT_SWIGLU: C is [M, N / 2]
     ep.act = act;
     ep.out_f32 = out_f32;
     ep.is_bf16 = is_bf16;

@@ -495,7 +495,8 @@ llm_argmax_kernel(float *__restrict__ logits, float *__restrict__ keep, int V_r,
             if (i < c1) {
                 if (keep) keep[(int64_t)b * V_r + i] = v[u];
                 row[i] = 0.f;
-                if (v[u] > best) { best = v[u]; bi = i; }   // ascending i: first maximum per thread
+                // ascending i: first maximum per thread (a strip of -inf still names its first element)
+                if (v[u] > best || (bi == 0x7fffffff && v[u] == best)) { best = v[u]; bi = i; }
             }
         }
     }
@@ -515,7 +516,7 @@ llm_argmax_kernel(float *__restrict__ logits, float *__restrict__ keep, int V_r,
     }
     if (threadIdx.x == 0) {
         // (value, index) -> one orderable 64-bit key: larger value first, then smaller index
-        const uint32_t fb = __float_as_uint(s_val[0]);
+        const uint32_t fb = __float_as_uint(s_val[0]) == 0x80000000u ? 0u : __float_as_uint(s_val[0]);   // -0.0 ties +0.0
         const uint32_t ord = (fb & 0x80000000u) ? ~fb : (fb | 0x80000000u);
         const unsigned long long key = ((unsigned long long)ord << 32) | (unsigned long long)(0xffffffffu - (uint32_t)s_idx[0]);
         atomicMax(row_key + b, key);
@@ -1394,6 +1395,76 @@ B2S_API int b2s_llm_flush_l2(b2s_llm *llm)
     if (!m) return fail(B2S_ERR_INVALID, "null argument");
     B2S_CUDA(cudaSetDevice(m->device));
     B2S_CUDA(cudaMemsetAsync(m->gu, 0, (size_t)256 << 20, m->stream));   // larger than the 126 MB L2
+    return 0;
+}
+
+// ---- operator-level entry points of the LLM kernels (device pointers): each calls the launcher the model itself uses
+B2S_API int b2s_op_llm_attn_decode(int device, void *cuda_stream, float *ws_qkv, void *k_pool, void *v_pool, int n_pages,
+                                   const int32_t *ctx_len, const int32_t *slots, const int32_t *page_table, int pages_per_seq,
+                                   const float *rope_cos, const float *rope_sin, int max_ctx, void *out, int n_seq, int n_heads,
+                                   int n_kv_heads, int stream_form, int n_cta, float *part_ws, int *part_cnt)
+{
+    using namespace b2s;
+    if (n_seq < 1 || n_seq > LLM_MAXB) return fail(B2S_ERR_INVALID, "llm decode attention: n_seq %d outside 1..%d", n_seq, LLM_MAXB);
+    if (n_kv_heads < 1 || n_pages < 1) return fail(B2S_ERR_INVALID, "llm decode attention: bad pool shape");
+    if (stream_form && (!part_ws || !part_cnt || n_cta < 1))
+        return fail(B2S_ERR_INVALID, "llm decode attention: the stream form needs part_ws, part_cnt and n_cta >= 1");
+    B2S_CUDA(cudaSetDevice(device));
+    CUtensorMap tk, tv;
+    if (stream_form) {
+        const int64_t rows = (int64_t)n_pages * n_kv_heads * 64;
+        B2S_TRY(make_tmap_2d_kmajor(&tk, k_pool, rows, LLM_HD, LLM_HD, 64, 1));
+        B2S_TRY(make_tmap_2d_kmajor(&tv, v_pool, rows, LLM_HD, LLM_HD, 64, 1));
+    }
+    return llm_attn_decode(static_cast<cudaStream_t>(cuda_stream), ws_qkv, k_pool, v_pool, ctx_len, slots, page_table, pages_per_seq,
+                           rope_cos, rope_sin, out, n_heads * LLM_HD, n_seq, n_heads, n_kv_heads, max_ctx, 1.0f / sqrtf((float)LLM_HD),
+                           stream_form ? &tk : nullptr, stream_form ? &tv : nullptr, part_ws, part_cnt, n_cta, stream_form);
+}
+
+B2S_API int b2s_op_llm_attn_prefill(int device, void *cuda_stream, void *qkv, void *k_pool, void *v_pool, const int32_t *cu_seqlens,
+                                    const int32_t *tok_seq, const int32_t *tok_pos, const int32_t *slots, const int32_t *page_table,
+                                    int pages_per_seq, const float *rope_cos, const float *rope_sin, int max_ctx, void *out, int n_seq,
+                                    int max_seqlen, int n_heads, int n_kv_heads)
+{
+    using namespace b2s;
+    if (n_seq < 1 || max_seqlen < 1 || n_kv_heads < 1 || n_heads % n_kv_heads)
+        return fail(B2S_ERR_INVALID, "llm prefill attention: bad shape");
+    B2S_CUDA(cudaSetDevice(device));
+    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    int32_t T = 0;   // one CTA per token for the RoPE + cache write: the token count is read back (this synchronises)
+    B2S_CUDA(cudaMemcpyAsync(&T, cu_seqlens + n_seq, 4, cudaMemcpyDeviceToHost, st));
+    B2S_CUDA(cudaStreamSynchronize(st));
+    if (T < 1) return fail(B2S_ERR_INVALID, "llm prefill attention: no tokens");
+    llm_rope_cache_prefill_kernel<<<T, 256, 0, st>>>(static_cast<__nv_bfloat16 *>(qkv), static_cast<__nv_bfloat16 *>(k_pool),
+                                                     static_cast<__nv_bfloat16 *>(v_pool), tok_seq, tok_pos, slots, page_table,
+                                                     pages_per_seq, rope_cos, rope_sin, n_heads, n_kv_heads, max_ctx);
+    count_launch();
+    B2S_CUDA(cudaGetLastError());
+    return llm_attn_prefill(st, qkv, (n_heads + 2 * n_kv_heads) * LLM_HD, k_pool, v_pool, cu_seqlens, slots, page_table, pages_per_seq,
+                            out, n_heads * LLM_HD, n_seq, max_seqlen, n_heads, n_kv_heads, 1.0f / sqrtf((float)LLM_HD));
+}
+
+B2S_API int b2s_op_llm_argmax(int device, void *cuda_stream, float *logits, float *keep, int n_seq, int vocab, int n_split,
+                              unsigned long long *row_key, int *row_cnt, int32_t *tokens)
+{
+    using namespace b2s;
+    if (n_seq < 1 || n_seq > 65535 || vocab < 1 || n_split < 1 || n_split > 65535)
+        return fail(B2S_ERR_INVALID, "llm argmax: bad shape");
+    B2S_CUDA(cudaSetDevice(device));
+    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    uint32_t *scratch = nullptr;   // [0]: step counter, [1, 1 + n_seq): output positions (all zero: no token buffer is written)
+    B2S_CUDA(cudaMalloc(&scratch, (size_t)(n_seq + 1) * 4));
+    cudaError_t e = cudaMemsetAsync(scratch, 0, (size_t)(n_seq + 1) * 4, st);
+    if (e == cudaSuccess) {
+        llm_argmax_kernel<<<dim3(n_seq, n_split), 256, 0, st>>>(logits, keep, vocab, 0, nullptr, nullptr, nullptr, nullptr, scratch, 0,
+                                                               tokens, nullptr, reinterpret_cast<const int32_t *>(scratch + 1), 0,
+                                                               row_key, row_cnt);
+        count_launch();
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    cudaFree(scratch);
+    B2S_CUDA(e);
     return 0;
 }
 

@@ -687,6 +687,12 @@ llm_attn_decode_stream_kernel(const __grid_constant__ CUtensorMap tmap_k, const 
         // in, fetches their partials WHILE it works on its own blocks and finishes the row without an arrival of its own --
         // no atomic and no dependent L2 round trip after the kernel's last block.  Anything else takes the arrival path below.
         const bool try_fast = (parts >= 2 && parts <= 4 && part == 0);
+        if (n_seg == 0) {
+            // QKV projection complete (q and the new k / v row are in ws_qkv) -- and with it every earlier kernel of the stream,
+            // among them the previous launch of this kernel: its arrivals on part_cnt must not be read as this launch's
+            griddep_wait();
+            if (warp == 1) LDS_STAMP(1);
+        }
         if (try_fast && ct == 0) {
             int seen;
             asm volatile("ld.acquire.gpu.global.s32 %0, [%1];\n" : "=r"(seen) : "l"(part_cnt + pkey) : "memory");
@@ -699,10 +705,6 @@ llm_attn_decode_stream_kernel(const __grid_constant__ CUtensorMap tmap_k, const 
         float *row = ws_qkv + (int64_t)b * QKV;
         // ---- prologue: RoPE on the group's q heads -> Qs; the new k / v row if this segment ends the sequence.
         // Every global load is issued before the first use: one L2 round trip per segment.
-        if (n_seg == 0) {
-            griddep_wait();             // QKV projection complete (q and the new k / v row are in ws_qkv)
-            if (warp == 1) LDS_STAMP(1);
-        }
         {
             const int i6 = ct & 63;
             constexpr int QIT = 512 / NC;       // G * 64 <= 512 (head, dim pair) items over NC threads

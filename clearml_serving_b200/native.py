@@ -128,6 +128,10 @@ PROTOTYPES = [
     ("b2s_llm_elapsed_ms", _i, [_vp, _i, _i, _P(ctypes.c_float)]),
     ("b2s_llm_flush_l2", _i, [_vp]),
     ("b2s_op_skinny_gemm", _i, [_i, _vp, _vp, _vp, _vp, _i, _i, _i]),
+    ("b2s_op_llm_attn_decode", _i, [_i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _i, _vp, _vp, _i, _vp, _i, _i, _i, _i, _i,
+                                    _vp, _vp]),
+    ("b2s_op_llm_attn_prefill", _i, [_i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _i, _vp, _i, _i, _i, _i]),
+    ("b2s_op_llm_argmax", _i, [_i, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
 ]
 
 _lib = None

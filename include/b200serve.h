@@ -200,7 +200,9 @@ B2S_API int b2s_timer_destroy(b2s_timer_t timer);
  * ONNX-Runtime backends (selected by triton_helper.py:378-385). */
 
 /* C[M,N] = act(A[M,K] . B[N,K]^T + bias[N]) + residual[M,N]; A,B,residual 16-bit (fp16 or bf16),
- * bias fp32, C 16-bit or fp32.  act: 0 none, 1 GELU(erf), 2 ReLU, 3 tanh.  tcgen05 + TMA + TMEM. */
+ * bias fp32, C 16-bit or fp32.  act: 0 none, 1 GELU(erf), 2 ReLU, 3 tanh, 4 SwiGLU (the LLM gate/up projection: columns
+ * [64j, 64j+32) of A.B^T are gate, [64j+32, 64j+64) up; C[M, N/2] 16-bit = silu(gate) * up, N % 64 == 0, no bias /
+ * residual).  tcgen05 + TMA + TMEM. */
 B2S_API int b2s_op_gemm(int device, void *cuda_stream, const void *A, const void *B, void *C, int M, int N,
                         int K, const float *bias, const void *residual, int act, int is_bf16, int out_f32);
 
@@ -309,6 +311,31 @@ B2S_API int b2s_llm_flush_l2(b2s_llm *llm);
 /* y[m][n_out] fp32 += X[m<=32, K] . W[n_out, K]^T (bf16 operands): the weight-streaming decode GEMM */
 B2S_API int b2s_op_skinny_gemm(int device, void *cuda_stream, const void *W, const void *X, float *y, int n_out,
                                int K, int m);
+/* Decode attention of one layer, fused with RoPE and the KV append (the kernels b2s_llm_decode runs).  ws_qkv fp32
+ * [n_seq, (n_heads + 2 n_kv_heads) * 128] is the QKV projection (q heads | k heads | v heads) and is left all zero;
+ * k_pool / v_pool bf16 [n_pages][n_kv_heads][64][128]; sequence b (<= 32) has ctx_len[b] cached tokens in the pages of
+ * page_table[slots[b] * pages_per_seq ...], its new k / v row is appended at position ctx_len[b] (clamped to max_ctx - 1);
+ * rope_cos / rope_sin fp32 [max_ctx][64]; out bf16 [n_seq, n_heads * 128].  stream_form 0: one CTA per (sequence, kv head);
+ * 1: 64-key blocks dealt over n_cta SMs (2 CTAs per SM when n_heads / n_kv_heads <= 4), partials in part_ws
+ * (2 * n_cta * 2 * 8 * 132 floats, no initial value needed) and arrival counters part_cnt (int [n_seq * n_kv_heads], zero
+ * before, left zero). */
+B2S_API int b2s_op_llm_attn_decode(int device, void *cuda_stream, float *ws_qkv, void *k_pool, void *v_pool, int n_pages,
+                                   const int32_t *ctx_len, const int32_t *slots, const int32_t *page_table, int pages_per_seq,
+                                   const float *rope_cos, const float *rope_sin, int max_ctx, void *out, int n_seq, int n_heads,
+                                   int n_kv_heads, int stream_form, int n_cta, float *part_ws, int *part_cnt);
+/* Prefill attention of one layer as b2s_llm_prefill runs it: RoPE on q (in place) and k, K / V rows written to the pages
+ * of each sequence's slot, then causal grouped-query attention.  qkv bf16 [T, (n_heads + 2 n_kv_heads) * 128];
+ * cu_seqlens int32 [n_seq + 1] (T = cu_seqlens[n_seq], read back: synchronises); token t is sequence tok_seq[t] at
+ * position tok_pos[t] (0, 1, ... within its sequence); out bf16 [T, n_heads * 128]. */
+B2S_API int b2s_op_llm_attn_prefill(int device, void *cuda_stream, void *qkv, void *k_pool, void *v_pool, const int32_t *cu_seqlens,
+                                    const int32_t *tok_seq, const int32_t *tok_pos, const int32_t *slots, const int32_t *page_table,
+                                    int pages_per_seq, const float *rope_cos, const float *rope_sin, int max_ctx, void *out, int n_seq,
+                                    int max_seqlen, int n_heads, int n_kv_heads);
+/* Greedy sampling: tokens[b] = index of the first maximum of logits fp32 [n_seq, vocab], the row split over n_split CTAs.
+ * logits are left zero, keep (or NULL) receives a copy; row_key / row_cnt ([n_seq], zero before) are left zero.
+ * Synchronises. */
+B2S_API int b2s_op_llm_argmax(int device, void *cuda_stream, float *logits, float *keep, int n_seq, int vocab, int n_split,
+                              unsigned long long *row_key, int *row_cnt, int32_t *tokens);
 
 #ifdef __cplusplus
 }

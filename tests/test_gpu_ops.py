@@ -6,14 +6,18 @@ import ctypes
 import numpy as np
 import pytest
 
+from clearml_serving_b200 import llm as L
+
 pytestmark = pytest.mark.gpu
 
 
 def _gemm(native, A, B, bias=None, residual=None, act=0, out_f32=False, bf16=False):
+    """A, B: fp16 arrays, or bf16 bit patterns (uint16) with bf16=True; returns C as float32 (fp32 or 16-bit output)"""
     M, K = A.shape
     N = B.shape[0]
+    n_out = N // 2 if act == 4 else N          # SwiGLU: C is [M, N / 2]
     dA, dB = native.DeviceBuffer(A.nbytes), native.DeviceBuffer(B.nbytes)
-    dC = native.DeviceBuffer(M * N * (4 if out_f32 else 2))
+    dC = native.DeviceBuffer(M * n_out * (4 if out_f32 else 2))
     dA.upload(A); dB.upload(B)
     dbias = dres = None
     if bias is not None:
@@ -24,11 +28,24 @@ def _gemm(native, A, B, bias=None, residual=None, act=0, out_f32=False, bf16=Fal
         native.check(native.lib().b2s_op_gemm(0, None, dA.ptr, dB.ptr, dC.ptr, M, N, K,
                                               dbias.ptr if dbias else None, dres.ptr if dres else None,
                                               act, 1 if bf16 else 0, 1 if out_f32 else 0))
-        return dC.download(np.float32 if out_f32 else np.float16, M * N).reshape(M, N)
+        if out_f32:
+            return dC.download(np.float32, M * n_out).reshape(M, n_out)
+        if bf16:
+            return L.from_bf16_bits(dC.download(np.uint16, M * n_out)).reshape(M, n_out)
+        return dC.download(np.float16, M * n_out).reshape(M, n_out).astype(np.float32)
     finally:
         for b in (dA, dB, dC, dbias, dres):
             if b is not None:
                 b.free()
+
+
+def _operand(rng, shape, std, dtype):
+    """random 16-bit GEMM operand: (what the kernel reads, its values as float32)"""
+    if dtype == "bf16":
+        bits = L.to_bf16_bits(rng.standard_normal(shape, dtype=np.float32) * np.float32(std))
+        return bits, L.from_bf16_bits(bits)
+    h = (rng.standard_normal(shape) * std).astype(np.float16)
+    return h, h.astype(np.float32)
 
 
 def _ref_act(x, act):
@@ -42,26 +59,57 @@ def _ref_act(x, act):
     return x
 
 
-@pytest.mark.parametrize("M,N,K", [(128, 128, 64), (128, 128, 768), (256, 768, 768), (300, 2304, 768),
-                                    (1000, 3072, 768), (77, 768, 3072), (5, 2, 768), (130, 200, 72), (260, 520, 136),
-                                    (4000, 256, 64), (20000, 768, 768),
-                                    # narrow, deep shapes (BERT FFN-down class): many k-blocks per tile, partly filled last wave
-                                    (7424, 768, 3072), (2000, 1024, 4096), (640, 512, 8192),
-                                    # 2-SM (cta_group::2) kernel: odd number of 128-row tiles (the last pair's second CTA is all
-                                    # padding), last 256-column tile partial
-                                    (4990, 1000, 2048),
-                                    # 256 x 192 pair-tiles (fp32 output, width a multiple of 192)
-                                    (4990, 960, 2048)])
-def test_gemm_fp16_matches_fp32_reference(gpu_native, M, N, K):
+GEMM_SHAPES = [(128, 128, 64), (128, 128, 768), (256, 768, 768), (300, 2304, 768),
+               (1000, 3072, 768), (77, 768, 3072), (5, 2, 768), (130, 200, 72), (260, 520, 136),
+               (4000, 256, 64), (20000, 768, 768),
+               # narrow, deep shapes (BERT FFN-down class): many k-blocks per tile, partly filled last wave
+               (7424, 768, 3072), (2000, 1024, 4096), (640, 512, 8192),
+               # 2-SM (cta_group::2) kernel: odd number of 128-row tiles (the last pair's second CTA is all
+               # padding), last 256-column tile partial
+               (4990, 1000, 2048),
+               # 256 x 192 pair-tiles (fp32 output, width a multiple of 192)
+               (4990, 960, 2048),
+               # LLM prefill projections (bf16): Llama-3-8B QKV at TP 1 and O, a ragged wave, a narrow one
+               (2048, 6144, 4096), (2000, 4096, 4096), (777, 1536, 512)]
+
+
+@pytest.mark.parametrize("M,N,K,dtype", [pytest.param(M, N, K, dt, id="{}-{}-{}{}".format(M, N, K, "" if dt == "fp16" else "-bf16"))
+                                         for dt in ("fp16", "bf16") for M, N, K in GEMM_SHAPES])
+def test_gemm_fp16_matches_fp32_reference(gpu_native, M, N, K, dtype):
     rng = np.random.default_rng(M * 7 + N)
-    A = (rng.standard_normal((M, K)) * 0.5).astype(np.float16)
-    B = (rng.standard_normal((N, K)) * 0.05).astype(np.float16)
-    ref = A.astype(np.float32) @ B.astype(np.float32).T
-    got = _gemm(gpu_native, A, B, out_f32=True)
-    # fp32 accumulation of exact fp16 products: only the summation order differs
+    A, A32 = _operand(rng, (M, K), 0.5, dtype)
+    B, B32 = _operand(rng, (N, K), 0.05, dtype)
+    bf = dtype == "bf16"
+    ref = A32 @ B32.T
+    got = _gemm(gpu_native, A, B, out_f32=True, bf16=bf)
+    # fp32 accumulation of exact 16-bit products: only the summation order differs
     np.testing.assert_allclose(got, ref, rtol=1e-4, atol=1e-4 * np.abs(ref).max())
-    got16 = _gemm(gpu_native, A, B).astype(np.float32)
-    np.testing.assert_allclose(got16, ref, rtol=2e-3, atol=2e-3 * np.abs(ref).max())
+    got16 = _gemm(gpu_native, A, B, bf16=bf)
+    tol = 8e-3 if bf else 2e-3                 # output rounding: 2^-9 (bf16) / 2^-11 (fp16) relative
+    np.testing.assert_allclose(got16, ref, rtol=tol, atol=tol * np.abs(ref).max())
+
+
+@pytest.mark.parametrize("M,N,dtype", [(M, N, "bf16") for N in (128, 192, 2048, 28672) for M in (1, 77, 300, 4096)]
+                         + [(300, 2048, "fp16")])
+def test_gemm_swiglu_epilogue(gpu_native, M, N, dtype):
+    """act 4, the prefill gate/up projection: fused columns [64j, 64j+32) are gate, [64j+32, 64j+64) up, C[M, N/2] =
+    silu(gate) * up.  Products above ~1e11 FLOP are checked on the first and last row of every 128-row tile plus
+    random rows."""
+    K = 4096 if N == 28672 else 512            # Llama-3-8B gate/up at TP 1: N = 2 * 14336, K = 4096
+    rng = np.random.default_rng(M + N)
+    A, A32 = _operand(rng, (M, K), 0.5, dtype)
+    B, B32 = _operand(rng, (N, K), 0.05, dtype)
+    got = _gemm(gpu_native, A, B, act=4, bf16=dtype == "bf16")
+    assert got.shape == (M, N // 2)
+    rows = np.arange(M)
+    if 2.0 * M * N * K > 1e11:
+        tiles = np.arange(0, M, 128)
+        rows = np.unique(np.concatenate([tiles, np.minimum(tiles + 127, M - 1), rng.integers(0, M, 64)]))
+    acc = (A32[rows] @ B32.T).astype(np.float64).reshape(len(rows), N // 64, 2, 32)
+    gate, up = acc[:, :, 0, :], acc[:, :, 1, :]
+    ref = (gate / (1.0 + np.exp(-gate)) * up).reshape(len(rows), N // 2)
+    tol = 8e-3 if dtype == "bf16" else 2e-3
+    np.testing.assert_allclose(got[rows], ref, rtol=tol, atol=tol * np.abs(ref).max())
 
 
 @pytest.mark.parametrize("act", [0, 1, 2, 3])
